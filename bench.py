@@ -48,7 +48,15 @@ def parse_args():
   ap.add_argument('--no-extras', action='store_true', help='skip the parity / precision1 / config4 / config5 blocks')
   ap.add_argument('--parity-sample', type=int, default=48, help='windows of the last timed step re-derived on the CPU oracle')
   ap.add_argument('--config5-windows', type=int, default=10_000_000)
-  return ap.parse_args()
+  ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                  help='write what the last timed step computed on rank 0 to DIR/<name>.npy as float32: probs.npy (every window, '
+                       'a fixed sample when over 2^20) and images.npy (a fixed sample of 48 windows); the same arguments give the same inputs')
+  args = ap.parse_args()
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
+  if args.dump_outputs and args.impl == 'reference':
+    ap.error('--dump-outputs writes the outputs of the CUDA path (--impl ours)')
+  return args
 
 
 def load_traffic():
@@ -327,6 +335,35 @@ def parity_block(params, tb, images, probs, weights_seed, n_sample, probs_p1=Non
   return out
 
 
+DUMP_IMAGES = 48                 # 48 x 100 x 221 x 7 float32 = 30 MB
+DUMP_MAX_PROB_ROWS = 1 << 20     # 12.6 MB of float32 probabilities
+
+
+def _seeded_rows(n, k, seed=0):
+  """All n rows when n <= k, else a fixed sorted sample of k of them."""
+  import numpy as np
+  if n <= k:
+    return np.arange(n)
+  return np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+
+
+def dump_outputs(out_dir, images, probs):
+  """Writes the last timed step's outputs, as a caller of the timed path receives them, to out_dir/<name>.npy in float32."""
+  import numpy as np
+  import torch
+  os.makedirs(out_dir, exist_ok=True)
+  arrays = {'images': (images, DUMP_IMAGES)}
+  if probs is not None:
+    arrays['probs'] = (probs, DUMP_MAX_PROB_ROWS)
+  shapes = {}
+  for name, (t, k) in arrays.items():
+    rows = torch.from_numpy(_seeded_rows(t.shape[0], k)).to(t.device)
+    a = t.index_select(0, rows).cpu().numpy().astype(np.float32)
+    np.save(os.path.join(out_dir, name + '.npy'), a)
+    shapes[name] = list(a.shape)
+  return shapes
+
+
 _REAL_STDOUT = None
 
 
@@ -417,6 +454,8 @@ def main():
   barrier()
   clocks = sampler.stop() if rank == 0 else None
   enc.check()
+  # Later blocks reuse `images` and `probs`: save the timed step's outputs before they run.
+  dumped = dump_outputs(args.dump_outputs, images, probs) if args.dump_outputs and rank == 0 else None
   ms_total = e0.elapsed_time(e1)
   launches = enc.launch_count + (cnn.launch_count if cnn else 0) - l0
   enc_ms = sum(a.elapsed_time(b) for a, b in enc_ev) / args.steps
@@ -632,6 +671,8 @@ def main():
       'gpu_launches': launches, 'clocks': clocks, 'e2e': e2e, 'roofline': roofline, 'roofline_encoder': roof_enc,
       'cpu_baseline': cpu_baseline,
   }
+  if dumped:
+    line['dump_outputs'] = {'dir': args.dump_outputs, 'arrays': dumped}
   line.update(extras)
   emit(line)
   if world > 1:

@@ -9,7 +9,7 @@ import pytest
 
 from deepvariant_b200 import _lib, bam
 
-REF_INPUT = '/root/reference/deepvariant/testdata/input'
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
 
 
 def _bgzf(payload: bytes, block=30000) -> bytes:
@@ -100,15 +100,18 @@ def test_rejects_garbage(tmp_path):
     bam.NativeBamTable(str(tmp_path / 'missing.bam'))
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_INPUT), reason='reference testdata is only present in the build container')
+# records at the head of each of the reference's test BAMs kept in tests/golden/reads_head.<name> (tools/make_reference_subset_fixtures.py)
+HEAD_RECORDS = {'NA12878_S1.chr20.10_10p1mb.bam': 400, 'test_pacbio.chr20_100kbp_at_9mb.bam': 16, 'HG002.hifi.hg37.phased.chr20.1_1000000.bam': 16}
+
+
 @pytest.mark.parametrize('name,aux', [('NA12878_S1.chr20.10_10p1mb.bam', False), ('test_pacbio.chr20_100kbp_at_9mb.bam', True),
                                      ('HG002.hifi.hg37.phased.chr20.1_1000000.bam', True)])
 def test_reference_testdata_identical_to_python_reader(name, aux):
-  """Every read of the reference's own test BAMs: the native table and the pure-Python reader agree field by field."""
-  path = os.path.join(REF_INPUT, name)
+  """The first records of the reference's own test BAMs, byte for byte: the native table and the pure-Python reader agree field by field."""
+  path = os.path.join(GOLDEN, 'reads_head.' + name)
   t = bam.NativeBamTable(path, parse_aux=aux)
   py = bam.BamReader(path, parse_aux=aux)
-  assert t.n_reads == len(py.reads) > 100
+  assert t.n_records_seen == HEAD_RECORDS[name] and t.n_reads == len(py.reads) > 0
   _same(t.reads(), py.reads)
   np.testing.assert_array_equal(t.end, np.array([r.end() for r in py.reads], dtype=np.int32))
 
@@ -127,17 +130,16 @@ def _assert_batches_equal(a, b):
     np.testing.assert_array_equal(a.arrays[k], b.arrays[k], err_msg=k)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_INPUT), reason='reference testdata is only present in the build container')
 def test_table_path_packs_the_same_batch_as_the_read_path_on_the_reference_candidates():
-  """The reference's 78 golden candidates over its NA12878 test BAM, partition by partition as make_examples walks
-  them: DvbBatch arrays from the table path (row numbers into the native read table) == arrays from Read objects."""
+  """The reference's 78 golden candidates over the reads of its NA12878 test BAM in chr20:9,999,000-10,011,000 (quickstart.chr20_10mb.bam,
+  a copy re-written with every read kept and the flags rebuilt), partition by partition as make_examples walks them: DvbBatch arrays from
+  the table path (row numbers into the native read table) == arrays from Read objects."""
   from deepvariant_b200 import fasta, packing, protos, tfrecord
-  td = os.path.dirname(REF_INPUT.rstrip('/')) + '/'
-  cands = [protos.parse_deepvariant_call(r) for r in tfrecord.read_records(td + 'golden.calling_candidates.tfrecord.gz')]
-  path = os.path.join(REF_INPUT, 'NA12878_S1.chr20.10_10p1mb.bam')
+  cands = [protos.parse_deepvariant_call(r) for r in tfrecord.read_records(os.path.join(GOLDEN, 'golden.calling_candidates.tfrecord.gz'))]
+  path = os.path.join(GOLDEN, 'quickstart.chr20_10mb.bam')
   req = bam.ReadRequirements(min_mapping_quality=5)
   reader, table = bam.BamReader(path, req), bam.NativeBamTable(path, req)
-  gen, params = _wgs_generator(fasta.IndexedFastaReader(os.path.join(REF_INPUT, 'ucsc.hg19.chr20.unittest.fasta.gz')))
+  gen, params = _wgs_generator(fasta.IndexedFastaReader(os.path.join(GOLDEN, 'quickstart.chr20_10mb.fa.gz')))
   region_start, part = 9_999_999, 1000
   by_part = {}
   for c in cands:
@@ -406,16 +408,16 @@ def test_region_restricted_open_equals_the_filtered_full_table(tmp_path):
   for c, s, e in (('chr1', 0, 1), ('chr1', 1000, 1500), ('chr2', 19990, 30000), ('chr2', 5000, 5001), ('chr1', 29999, 30000)):
     rid = full.references.index(c)
     np.testing.assert_array_equal(full.query_indices(c, s, e), np.nonzero((full.ref_id == rid) & (full.pos < e) & (full.end > s))[0])
-  real = '/root/reference/deepvariant/testdata/input/NA12878_S1.chr20.10_10p1mb.bam'
-  if os.path.exists(real) and os.path.exists(real + '.bai'):
-    full = bam.NativeBamTable(real, reqs)
-    for s, e in ((10_000_000, 10_010_000), (10_050_123, 10_050_124), (10_099_000, 10_100_000), (9_000_000, 9_500_000)):
-      rid = full.references.index('chr20')
-      keep = (full.ref_id == rid) & (full.pos < e) & (full.end > s)
-      sub = bam.NativeBamTable(real, reqs, regions=[('chr20', s, e)])
-      _assert_same_rows(sub, full, keep)
-      if keep.any() and s > 10_020_000:
-        assert sub.n_records_seen < full.n_records_seen // 2, 'the index was not used: the whole file was parsed'
+  # real reads: the records of the reference's NA12878 test BAM that start before chr20:10,011,000, with their .bai
+  real = os.path.join(GOLDEN, 'NA12878_S1.chr20.10_10p1mb.window.bam')
+  full = bam.NativeBamTable(real, reqs)
+  for s, e in ((10_000_000, 10_010_000), (10_005_123, 10_005_124), (10_010_700, 10_011_000), (9_000_000, 9_500_000)):
+    rid = full.references.index('chr20')
+    keep = (full.ref_id == rid) & (full.pos < e) & (full.end > s)
+    sub = bam.NativeBamTable(real, reqs, regions=[('chr20', s, e)])
+    _assert_same_rows(sub, full, keep)
+    if keep.any() and s > 10_010_624:      # past the first 16-kb window of the linear index the file holds reads of
+      assert sub.n_records_seen < full.n_records_seen // 2, 'the index was not used: the whole file was parsed'
 
 
 def test_malformed_bgzf_headers_are_rejected_not_overrun(tmp_path):

@@ -5,7 +5,7 @@
     native table) and against the Python restatement oracle/candidates_oracle.py;
   * product == oracle on random reads (indels, clips, N bases, low qualities, repeated read keys, track_ref_reads);
   * the reference's golden files: a portable fixture cut from golden.calling_candidates (tools/check_candidates_golden.py)
-    and, where /root/reference exists, all of golden.calling_candidates / golden.pacbio_examples.
+    and the variants of golden.pacbio_examples in a 5-kb window (tools/make_reference_subset_fixtures.py).
 CPU-only: host code of libdvb.so."""
 import json
 import os
@@ -22,7 +22,6 @@ import test_bam_native as tb  # noqa: E402
 from deepvariant_b200 import bam, candidates as cand, protos  # noqa: E402
 
 GOLDEN = os.path.join(ROOT, 'tests', 'golden')
-TESTDATA = '/root/reference/deepvariant/testdata'
 # third_party/nucleus/testdata/test.fasta, the contigs allelecounter_test.cc uses
 CHR1 = b'ACCACCATCCTCCGTGAAATCAATATCCCGCACAAGAGTGCTACTCTCCTAAATCCCTTCTCGTCCCCATGGATGA'
 CHR2 = b'CGCTNCGGGCCCATAACACTTGGGGGTAGCTAAAGTGAACTGTATCC'
@@ -442,13 +441,16 @@ def test_golden_fixture_candidates_reproduced(tmp_path):
   assert n >= 8
 
 
-@pytest.mark.skipif(not os.path.isdir(TESTDATA), reason='reference testdata is only present in the build container')
 def test_pacbio_golden_variants_all_reproduced():
-  """golden.pacbio_examples (realigner off): 341 of 341 variants identical in site, alleles, AD, DP, VAF; none extra."""
+  """golden.pacbio_examples (realigner off) in chr20:9,060,000-9,065,000, from the reads of the reference's PacBio test BAM that overlap it
+  (tests/golden/, tools/make_reference_subset_fixtures.py): 12 of 12 variants identical in site, alleles, AD, DP, VAF; none extra.
+  All 341 of the whole 100 kb are pinned by tests/golden/candidates_golden_report.json."""
   sys.path.insert(0, os.path.join(ROOT, 'tools'))
   import check_candidates_golden as ck
-  r = ck.pacbio_pin()
-  assert r['golden_variants'] == r['ours_candidates'] == r['identical_site_alleles_AD_DP_VAF'] == 341
+  window = 'chr20_9060000_9065000'
+  r = ck.pacbio_pin(os.path.join(GOLDEN, f'test_pacbio.{window}.bam'), os.path.join(GOLDEN, 'grch38.chr20_9030000_9135000.fa.gz'),
+                    json.load(open(os.path.join(GOLDEN, f'golden.pacbio_variants.{window}.json'))), ('chr20', 9_060_000, 9_065_000))
+  assert r['golden_variants'] == r['ours_candidates'] == r['identical_site_alleles_AD_DP_VAF'] == 12
   assert r['golden_only'] == r['ours_only'] == 0
 
 

@@ -1,5 +1,5 @@
 """CRAM 3.0 input (csrc/dvb_cram.cu -> dvb_cram_to_bam): the reference's own small CRAM vectors (tests/golden/cram/, copied by
-tools/make_cram_fixtures.py) against the SAM they were written from, and - in the build container - the reference's chr20 CRAM against
+tools/make_cram_fixtures.py) against the SAM they were written from, and the first container of the reference's chr20 CRAM against
 its BAM, read for read (make_examples_test.py:330-372 expects the BAM's goldens from that CRAM)."""
 import os
 import sys
@@ -11,8 +11,13 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from deepvariant_b200 import _lib, bam, candidates as cand, fasta  # noqa: E402
 
-CRAM = os.path.join(ROOT, 'tests', 'golden', 'cram')
-REF_INPUT = '/root/reference/deepvariant/testdata/input'
+GOLDEN = os.path.join(ROOT, 'tests', 'golden')
+CRAM = os.path.join(GOLDEN, 'cram')
+# The reference's chr20 CRAM cut to its first container (10,000 records from chr20:9,999,912), the records of its BAM that start
+# before chr20:10,011,000, and the reference bases of chr20:9,990,000-10,020,000 (tools/make_reference_subset_fixtures.py).
+CHR20_CRAM = os.path.join(GOLDEN, 'NA12878_S1.chr20.10_10p1mb.first_container.cram')
+CHR20_BAM = os.path.join(GOLDEN, 'NA12878_S1.chr20.10_10p1mb.window.bam')
+CHR20_FASTA = os.path.join(GOLDEN, 'quickstart.chr20_10mb.fa.gz')
 
 
 def _keep_all():
@@ -98,38 +103,39 @@ def test_cram_argument_errors(tmp_path):
     assert rc in (0, 1, 7)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_INPUT), reason='reference testdata is only present in the build container')
 def test_reference_chr20_cram_equals_its_bam_read_for_read():
-  """52,035 records, gzip and rANS (order 0 and 1) blocks, mates linked inside slices and detached ones: every field the table holds."""
-  ref = fasta.IndexedFastaReader(os.path.join(REF_INPUT, 'ucsc.hg19.chr20.unittest.fasta.gz'))
-  c = bam.NativeBamTable(os.path.join(REF_INPUT, 'NA12878_S1.chr20.10_10p1mb.cram'), _keep_all(), parse_aux=True, ref_reader=ref)
-  b = bam.NativeBamTable(os.path.join(REF_INPUT, 'NA12878_S1.chr20.10_10p1mb.bam'), _keep_all(), parse_aux=True)
-  assert c.n_reads == b.n_reads == 52035
+  """The reads of the CRAM's first container that start before chr20:10,010,000 against the same reads of the BAM: gzip and rANS
+  (order 0 and 1) blocks, mates linked inside the slices and detached ones, every field the table holds."""
+  ref = fasta.IndexedFastaReader(CHR20_FASTA)
+  assert bam.NativeBamTable(CHR20_CRAM, _keep_all(), ref_reader=ref).n_reads == 10000
+  whole = [('chr20', 0, 10_010_000)]       # every read of the BAM fixture starting before 10,010,000, and no read past the container
+  c = bam.NativeBamTable(CHR20_CRAM, _keep_all(), parse_aux=True, ref_reader=ref, regions=whole)
+  b = bam.NativeBamTable(CHR20_BAM, _keep_all(), parse_aux=True, regions=whole)
+  assert c.n_reads == b.n_reads == 4986
   for name in ('ref_id', 'pos', 'end', 'mapq', 'flag', 'fragment_length', 'hp', 'read_number', 'number_reads', 'seq_begin', 'cigar_begin', 'name_begin',
                'bases', 'quals', 'cigar'):
     np.testing.assert_array_equal(getattr(c, name), getattr(b, name), err_msg=name)
   assert c.names == b.names
-  # a region-restricted open decodes only the containers it needs and gives the rows the BAM's region open gives
-  regions = [('chr20', 10050000, 10051000)]
-  cr = bam.NativeBamTable(os.path.join(REF_INPUT, 'NA12878_S1.chr20.10_10p1mb.cram'), _keep_all(), ref_reader=ref, regions=regions)
-  br = bam.NativeBamTable(os.path.join(REF_INPUT, 'NA12878_S1.chr20.10_10p1mb.bam'), _keep_all(), regions=regions)
+  # a region-restricted open gives the rows the BAM's region open gives
+  regions = [('chr20', 10005000, 10006000)]
+  cr = bam.NativeBamTable(CHR20_CRAM, _keep_all(), ref_reader=ref, regions=regions)
+  br = bam.NativeBamTable(CHR20_BAM, _keep_all(), regions=regions)
   assert cr.n_reads == br.n_reads > 100 and cr.reads() == br.reads()
-  assert cand.sample_name_from_bam(os.path.join(REF_INPUT, 'NA12878_S1.chr20.10_10p1mb.cram')) == 'NA12878'
+  assert cand.sample_name_from_bam(CHR20_CRAM) == 'NA12878'
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_INPUT), reason='reference testdata is only present in the build container')
 def test_make_examples_over_the_cram_writes_the_goldens_of_the_bam(tmp_path, monkeypatch):
   """make_examples_test.py:330-372 (TestConditions.USE_CRAM): --reads NA12878_S1.chr20.10_10p1mb.cram must give golden.calling_examples.
-  The encoder is the CPU oracle here (no GPU in the build container); reads, realigner, candidates and planning are the product flow."""
+  The encoder is the CPU oracle here; reads, realigner, candidates and planning are the product flow."""
   sys.path.insert(0, os.path.join(ROOT, 'tests'))
   import test_candidates as tc
   from deepvariant_b200 import cli, make_examples_native as men, pileup_image as pi, protos, tfrecord
   monkeypatch.setattr(men.ExamplesGenerator, '_gpu', lambda self: tc.OracleEncoder(pi.to_params(self.options.pic_options, height=self.pileup_image_height)))
   out = str(tmp_path / 'examples.tfrecord.gz')
-  assert cli.make_examples(['--mode', 'calling', '--ref', os.path.join(REF_INPUT, 'ucsc.hg19.chr20.unittest.fasta.gz'),
-                            '--reads', os.path.join(REF_INPUT, 'NA12878_S1.chr20.10_10p1mb.cram'), '--regions', 'chr20:10,000,000-10,010,000',
+  assert cli.make_examples(['--mode', 'calling', '--ref', CHR20_FASTA,
+                            '--reads', CHR20_CRAM, '--regions', 'chr20:10,000,000-10,010,000',
                             '--examples', out, '--channel_list', 'BASE_CHANNELS,insert_size']) == 0
-  golden = [protos.parse_tf_example(r) for r in tfrecord.read_records(os.path.join(os.path.dirname(REF_INPUT), 'golden.calling_examples.tfrecord.gz'))]
+  golden = [protos.parse_tf_example(r) for r in tfrecord.read_records(os.path.join(GOLDEN, 'golden.calling_examples.tfrecord.gz'))]
   ours = [protos.parse_tf_example(r) for r in tfrecord.read_records(out)]
   assert len(ours) == len(golden) == 84
   for g, o in zip(golden, ours):

@@ -1,8 +1,9 @@
 """Local realigner (deepvariant_b200/realigner.py): window selector, de Bruijn graph, assembly + FastPassAligner.
 
 Known answers transcribed from deepvariant/realigner/window_selector_test.py:455-540 and python/debruijn_graph_wrap_test.py:80-360;
-where /root/reference exists, the reference's WGS goldens - made WITH the realigner - end to end: 78 of 78 golden candidates identical
-in every field and 84 of 84 golden.calling_examples images byte for byte (tools/check_realigner_golden.py).  CPU-only."""
+the reference's WGS goldens - made WITH the realigner - end to end from the reads of its NA12878 test BAM that start before
+chr20:10,011,000 (tests/golden/, tools/make_reference_subset_fixtures.py): 78 of 78 golden candidates identical in every field and 84 of
+84 golden.calling_examples images byte for byte (tools/check_realigner_golden.py).  CPU-only."""
 import json
 import os
 import sys
@@ -13,6 +14,9 @@ from deepvariant_b200 import realigner as rl
 from deepvariant_b200.protos import Read
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+GOLDEN = os.path.join(ROOT, 'tests', 'golden')
+# the reference bases of chr20:9,990,000-10,020,000, where the reads of the window BAM lie
+QUICKSTART_FASTA = os.path.join(GOLDEN, 'quickstart.chr20_10mb.fa.gz')
 
 
 def _read(seq, pos=1, qual=30, mapq=60):
@@ -69,12 +73,11 @@ def test_variant_reads_candidate_positions():
   assert got == [1003] + [1006, 1007, 1008, 1009] + [1012, 1013]
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/deepvariant/testdata'), reason='reference testdata is only present in the build container')
 def test_wgs_goldens_made_with_the_realigner_are_reproduced_end_to_end():
   sys.path.insert(0, os.path.join(ROOT, 'tools'))
   import check_realigner_golden
-  check_realigner_golden.main()
-  r = json.load(open(os.path.join(ROOT, 'tests/golden/realigner_golden_report.json')))
+  r = check_realigner_golden.main(td=GOLDEN, bam_path=os.path.join(GOLDEN, 'NA12878_S1.chr20.10_10p1mb.window.bam'), ref_path=QUICKSTART_FASTA,
+                                  shard_keys=json.load(open(os.path.join(GOLDEN, 'golden.calling_examples.shard_keys.json'))), write=False)
   assert r['golden_candidates'] == r['ours_candidates'] == r['candidates_identical_in_every_field'] == 78
   assert r['golden_examples'] == r['examples_planned'] == r['images_identical'] == 84
   assert r['golden_read_rows'] == r['golden_read_rows_reproduced'] == 4309
@@ -87,13 +90,14 @@ def test_realigner_report_is_committed():
   assert r['candidates_identical_in_every_field'] == 78 and r['images_identical'] == 84
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/deepvariant/testdata'), reason='reference testdata is only present in the build container')
 def test_wgs_alt_aligned_goldens_diff_channels_and_rows():
-  """golden.alt_aligned_pileup_{diff_channels,rows}_examples: 49 of 49 images each (100 x 221 x 8 / 300 x 221 x 6), realigner on."""
+  """golden.alt_aligned_pileup_{diff_channels,rows}_examples: 49 of 49 images each (100 x 221 x 8 / 300 x 221 x 6), realigner on;
+  the golden images are held as SHA-256 digests (golden.alt_aligned_pileup.digests.json)."""
   sys.path.insert(0, os.path.join(ROOT, 'tools'))
   import check_alt_aligned_wgs_golden
-  check_alt_aligned_wgs_golden.main()
-  for r in json.load(open(os.path.join(ROOT, 'tests/golden/alt_aligned_wgs_report.json'))):
+  digests = json.load(open(os.path.join(GOLDEN, 'golden.alt_aligned_pileup.digests.json')))
+  for layout in ('diff_channels', 'rows'):
+    r = check_alt_aligned_wgs_golden.run(layout, digests[layout], os.path.join(GOLDEN, 'NA12878_S1.chr20.10_10p1mb.window.bam'), QUICKSTART_FASTA)
     assert r['compared'] == r['images_identical'] == r['golden_examples'] == 49 and r['of_those_identical'] == r['examples_with_alt_aligned_pileups'] == 4
 
 

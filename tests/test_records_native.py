@@ -12,7 +12,7 @@ from hypothesis import given, settings, strategies as st
 
 from deepvariant_b200 import _lib, call_variants as cv, protos, records, tfrecord
 
-REF_TESTDATA = '/root/reference/deepvariant/testdata'
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
 
 
 def _example(image: bytes, variant: bytes, alt: bytes, shape=(2, 3, 1), extra=True) -> bytes:
@@ -158,9 +158,8 @@ def test_reader_errors(tmp_path):
         r.next_into(np.zeros((2, 6), dtype=np.uint8))
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_TESTDATA), reason='reference testdata is only present in the build container')
 def test_reader_on_the_reference_golden_examples():
-  path = os.path.join(REF_TESTDATA, 'golden.calling_examples.tfrecord.gz')
+  path = os.path.join(GOLDEN, 'golden.calling_examples.tfrecord.gz')
   want = [protos.parse_tf_example(r) for r in tfrecord.read_records(path)]
   with records.NativeExamplesReader([path]) as r:
     shape, nbytes = r.shape()

@@ -2,6 +2,7 @@
 training mode over chr20:10,000,000-10,010,000 with the realigner; training only drops / labels examples, the images of the examples it
 keeps are those of calling mode).  Every golden example is rebuilt from BAM + FASTA: realigner -> candidates -> pileups + alt-aligned
 pileups -> diff channels (100 x 221 x 8) or stacked rows (300 x 221 x 6).  Writes tests/golden/alt_aligned_wgs_report.json."""
+import hashlib
 import json
 import os
 import sys
@@ -20,15 +21,24 @@ from deepvariant_b200 import pileup_image as pi  # noqa: E402
 T = '/root/reference/deepvariant/testdata/'
 
 
-def run(layout: str) -> dict:
+def image_digest(image: bytes, shape) -> str:
+  """SHA-256 of an example's image bytes and shape."""
+  return hashlib.sha256(bytes(image) + repr([int(x) for x in shape]).encode()).hexdigest()
+
+
+def run(layout: str, golden_digests=None, bam_path=None, ref_path=None) -> dict:
+  """golden_digests: [start, alt allele indices, image_digest] per golden example (default: read from the testdata's goldens)."""
   golden = {}
-  for r in tfrecord.read_records(T + f'golden.alt_aligned_pileup_{layout}_examples.tfrecord.gz'):
-    e = protos.parse_tf_example(r)
-    v = protos.parse_variant(e['variant/encoded'][1][0])
-    golden[(v.start, tuple(protos.parse_alt_allele_indices(e['alt_allele_indices/encoded'][1][0])))] = \
-        np.frombuffer(e['image/encoded'][1][0], np.uint8).reshape(e['image/shape'][1])
-  ref = fasta.IndexedFastaReader(T + 'input/ucsc.hg19.chr20.unittest.fasta.gz')
-  table = bam.NativeBamTable(T + 'input/NA12878_S1.chr20.10_10p1mb.bam', bam.ReadRequirements(min_mapping_quality=5))
+  if golden_digests is None:
+    golden_digests = []
+    for r in tfrecord.read_records(T + f'golden.alt_aligned_pileup_{layout}_examples.tfrecord.gz'):
+      e = protos.parse_tf_example(r)
+      golden_digests.append([protos.parse_variant(e['variant/encoded'][1][0]).start, protos.parse_alt_allele_indices(e['alt_allele_indices/encoded'][1][0]),
+                             image_digest(e['image/encoded'][1][0], e['image/shape'][1])])
+  for start, idx, digest in golden_digests:
+    golden[(start, tuple(idx))] = digest
+  ref = fasta.IndexedFastaReader(ref_path or T + 'input/ucsc.hg19.chr20.unittest.fasta.gz')
+  table = bam.NativeBamTable(bam_path or T + 'input/NA12878_S1.chr20.10_10p1mb.bam', bam.ReadRequirements(min_mapping_quality=5))
   copts = cand.CandidateOptions(sample_name='NA12878')
   pic = pi.default_options(pi.ReadRequirements(10, 5))
   pic.channels = list(pi.PILEUP_DEFAULT_CHANNELS)
@@ -40,7 +50,7 @@ def run(layout: str) -> dict:
   params = pi.to_params(pic)
   rl = realigner.Realigner(ref)
   refs = [(c, ref.n_bases(c)) for c in ref.contig_order]
-  stats = dict(layout=layout, golden_examples=len(golden), shape=list(next(iter(golden.values())).shape), compared=0, images_identical=0,
+  stats = dict(layout=layout, golden_examples=len(golden), shape=list(gen.image_shape()), compared=0, images_identical=0,
                examples_with_alt_aligned_pileups=0, of_those_identical=0)
   with tempfile.TemporaryDirectory() as tmp:
     for contig, s, e in cand.regions_to_process(refs, 1000, ('chr20', 9999999, 10010000)):
@@ -65,7 +75,7 @@ def run(layout: str) -> dict:
         g = golden.get((p.variant.start, tuple(p.variant.alternate_bases.index(a) for a in p.alt_combination)))
         if g is None:
           continue          # training mode dropped it (outside the confident regions)
-        ok = bool(np.array_equal(img, g))
+        ok = image_digest(np.ascontiguousarray(img).tobytes(), img.shape) == g
         stats['compared'] += 1
         stats['images_identical'] += ok
         if p.alt_specs:

@@ -64,26 +64,36 @@ def main():
   write_fixture(fixture, g_by, o_by, table, ref, opts)
 
 
-def pacbio_pin():
-  """golden.pacbio_examples.tfrecord.gz (make_examples_test.py:792-831: realigner off, --track_ref_reads, --phase_reads region
-  padding, --vsc_min_fraction_indels 0.12, --partition_size 25000): every variant/encoded of the 401 examples against ours."""
-  examples = [protos.parse_tf_example(r) for r in tfrecord.read_records(os.path.join(TESTDATA, 'golden.pacbio_examples.tfrecord.gz'))]
+def pacbio_golden_variants(path: str) -> dict:
+  """The variants of golden.pacbio_examples, by (start, ref, alts)."""
   gold = {}
-  for e in examples:
-    c = canonical(protos.f_bytes(1, e['variant/encoded'][1][0]))
+  for r in tfrecord.read_records(path):
+    c = canonical(protos.f_bytes(1, protos.parse_tf_example(r)['variant/encoded'][1][0]))
     gold[(c['start'], c['ref'], tuple(c['alts']))] = c
-  bam_path = os.path.join(TESTDATA, 'input/test_pacbio.chr20_100kbp_at_9mb.bam')
-  ref = fasta.IndexedFastaReader(os.path.join(TESTDATA, 'input/grch38.chr20_and_21_10M.fa.gz'))
+  return gold
+
+
+def pacbio_pin(bam_path=None, ref_path=None, golden=None, region=('chr20', 8999999, 9100000)):
+  """golden.pacbio_examples.tfrecord.gz (make_examples_test.py:792-831: realigner off, --track_ref_reads, --phase_reads region
+  padding, --vsc_min_fraction_indels 0.12, --partition_size 25000): every variant/encoded of the 401 examples against ours.
+  golden: canonical_call dicts of the golden variants (default: all of golden.pacbio_examples); region: where to call them."""
+  if golden is None:
+    gold = pacbio_golden_variants(os.path.join(TESTDATA, 'golden.pacbio_examples.tfrecord.gz'))
+  else:
+    gold = {(c['start'], c['ref'], tuple(c['alts'])): c for c in golden}
+  bam_path = bam_path or os.path.join(TESTDATA, 'input/test_pacbio.chr20_100kbp_at_9mb.bam')
+  ref = fasta.IndexedFastaReader(ref_path or os.path.join(TESTDATA, 'input/grch38.chr20_and_21_10M.fa.gz'))
   table = bam.NativeBamTable(bam_path, bam.ReadRequirements(min_mapping_quality=1), parse_aux=True)
   opts = cand.CandidateOptions(sample_name=cand.sample_name_from_bam(bam_path), min_mapping_quality=1, track_ref_reads=True,
                                vsc_min_fraction_indels=0.12, partition_size=25000)
   ours = {}
-  for contig, s, e in cand.regions_to_process([(c, ref.n_bases(c)) for c in ref.contig_order], 25000, ('chr20', 8999999, 9100000)):
+  for contig, s, e in cand.regions_to_process([(c, ref.n_bases(c)) for c in ref.contig_order], 25000, region):
     for rec in cand.candidates_in_region(table, ref, contig, s, e, opts, padding_pct=20).records:
       c = canonical(rec)
       ours[(c['start'], c['ref'], tuple(c['alts']))] = c
   same = [k for k in gold if k in ours and all(gold[k][f] == ours[k][f] for f in ('info', 'call_set_name', 'genotype', 'end', 'contig'))]
-  return {'golden_examples': len(examples), 'golden_variants': len(gold), 'ours_candidates': len(ours),
+  n_examples = sum(1 for _ in tfrecord.read_records(os.path.join(TESTDATA, 'golden.pacbio_examples.tfrecord.gz'))) if golden is None else None
+  return {'golden_examples': n_examples, 'golden_variants': len(gold), 'ours_candidates': len(ours),
           'identical_site_alleles_AD_DP_VAF': len(same), 'golden_only': len(set(gold) - set(ours)), 'ours_only': len(set(ours) - set(gold))}
 
 

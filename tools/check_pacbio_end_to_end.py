@@ -17,24 +17,44 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, 'tests'))
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 import oracle_lib  # noqa: E402
 from deepvariant_b200 import bam, candidates as cand, direct_phasing, fasta, packing, protos, tfrecord  # noqa: E402
 from deepvariant_b200 import make_examples_native as men  # noqa: E402
 from deepvariant_b200 import pileup_image as pi  # noqa: E402
 
 T = '/root/reference/deepvariant/testdata/'
+REGION = ('chr20', 8999999, 9100000)
 
 
-def main():
-  examples = [protos.parse_tf_example(r) for r in tfrecord.read_records(T + 'golden.pacbio_examples.tfrecord.gz')]
-  golden = {}
-  for e in examples:
-    v = protos.parse_variant(e['variant/encoded'][1][0])
-    idx = tuple(protos.parse_alt_allele_indices(e['alt_allele_indices/encoded'][1][0]))
-    golden[(v.start, idx)] = np.frombuffer(e['image/encoded'][1][0], dtype=np.uint8).reshape(e['image/shape'][1])
-  bam_path = T + 'input/test_pacbio.chr20_100kbp_at_9mb.bam'
+def channel_summary(img: np.ndarray) -> dict:
+  """Per channel of an example image: SHA-256 of its pixels and whether any is set; and its non-blank read rows."""
+  from check_alt_aligned_wgs_golden import image_digest
+  chans = [np.ascontiguousarray(img[..., c]) for c in range(img.shape[-1])]
+  return {'digests': [image_digest(c.tobytes(), c.shape) for c in chans], 'nonzero': [bool(c.any()) for c in chans],
+          'rows': int(sum(1 for r in range(5, img.shape[0]) if img[r].any()))}
+
+
+def golden_summaries(path: str) -> list:
+  """[start, alt allele indices, channel_summary] per example of a golden examples file."""
+  out = []
+  for r in tfrecord.read_records(path):
+    e = protos.parse_tf_example(r)
+    img = np.frombuffer(e['image/encoded'][1][0], dtype=np.uint8).reshape(e['image/shape'][1])
+    out.append([protos.parse_variant(e['variant/encoded'][1][0]).start, protos.parse_alt_allele_indices(e['alt_allele_indices/encoded'][1][0]),
+                channel_summary(img)])
+  return out
+
+
+def main(bam_path=None, ref_path=None, golden=None, region=REGION, write=True):
+  """golden: golden_summaries of the examples to compare with (default: all of the testdata's golden.pacbio_examples); region: the
+  part of chr20 to make examples for, in 25-kb partitions from its start.  Returns the stats."""
+  if golden is None:
+    golden = golden_summaries(T + 'golden.pacbio_examples.tfrecord.gz')
+  golden = {(start, tuple(idx)): g for start, idx, g in golden}
+  bam_path = bam_path or T + 'input/test_pacbio.chr20_100kbp_at_9mb.bam'
   table = bam.NativeBamTable(bam_path, bam.ReadRequirements(min_mapping_quality=1), parse_aux=True)
-  ref = fasta.IndexedFastaReader(T + 'input/grch38.chr20_and_21_10M.fa.gz')
+  ref = fasta.IndexedFastaReader(ref_path or T + 'input/grch38.chr20_and_21_10M.fa.gz')
   copts = cand.CandidateOptions(sample_name=cand.sample_name_from_bam(bam_path), min_mapping_quality=1, track_ref_reads=True,
                                 vsc_min_fraction_indels=0.12, partition_size=25000)
   pic = pi.default_options(pi.ReadRequirements(min_base_quality=10, min_mapping_quality=1))
@@ -48,7 +68,7 @@ def main():
   stats = dict(examples=0, images_equal_7_channels=0, haplotype_channel_equal=0, row_order_equal=0, reads_phased=0, reads=0, snp_examples=0,
                snp_alt_aligned_channels_zero_in_golden=0, methylation_channel_zero=0)
   mismatches = []
-  for contig, s, e in cand.regions_to_process([(c, ref.n_bases(c)) for c in ref.contig_order], 25000, ('chr20', 8999999, 9100000)):
+  for contig, s, e in cand.regions_to_process([(c, ref.n_bases(c)) for c in ref.contig_order], 25000, region):
     rows = cand.region_reads(table, contig, s, e, copts.max_reads_per_partition, copts.random_seed)
     found = cand.candidates_in_region(table, ref, contig, s, e, copts, rows=rows, padding_pct=20)
     reads = [table.read(int(r)) for r in rows]                      # fresh Read objects for this region, like a new BAM query
@@ -71,34 +91,36 @@ def main():
       if g is None:
         mismatches.append({'start': p.variant.start, 'why': 'not in golden'})
         continue
+      o = channel_summary(img)
+      same = [a == b for a, b in zip(o['digests'], g['digests'])]
       stats['examples'] += 1
-      eq7 = bool(np.array_equal(img[..., :7], g[..., :7]))
+      eq7 = all(same[:7])
       stats['images_equal_7_channels'] += eq7
-      stats['haplotype_channel_equal'] += bool(np.array_equal(img[..., 6], g[..., 6]))
-      stats['row_order_equal'] += bool(np.array_equal(img[..., :4], g[..., :4]))
-      stats['methylation_channel_zero'] += bool(not g[..., 7].any())
-      alt_eq = bool(np.array_equal(img[..., 8:10], g[..., 8:10]))
+      stats['haplotype_channel_equal'] += same[6]
+      stats['row_order_equal'] += all(same[:4])
+      stats['methylation_channel_zero'] += not g['nonzero'][7]
+      alt_eq = all(same[8:10])
       stats['alt_aligned_channels_equal'] = stats.get('alt_aligned_channels_equal', 0) + alt_eq
-      stats['whole_image_equal'] = stats.get('whole_image_equal', 0) + bool(np.array_equal(img, g))   # all ten channels, the golden's own layout
+      stats['whole_image_equal'] = stats.get('whole_image_equal', 0) + all(same)   # all ten channels, the golden's own layout
       if p.variant_type != 1:
         stats['indel_examples'] = stats.get('indel_examples', 0) + 1
         stats['indel_alt_aligned_channels_equal'] = stats.get('indel_alt_aligned_channels_equal', 0) + alt_eq
         if not alt_eq and len(mismatches) < 40:
-          d = (img[..., 8:10] != g[..., 8:10])
-          mismatches.append({'start': p.variant.start, 'alts': p.alt_combination, 'alt_channel_pixels_differ': int(d.sum()),
-                             'rows_differ': int(d.any(axis=(1, 2)).sum()), 'rows': int(sum(1 for r in range(5, 100) if g[r].any()))})
+          mismatches.append({'start': p.variant.start, 'alts': p.alt_combination, 'alt_channels_differ': [c for c in (8, 9) if not same[c]],
+                             'rows': g['rows']})
       if p.variant_type == 1:
         stats['snp_examples'] += 1
-        stats['snp_alt_aligned_channels_zero_in_golden'] += bool(not g[..., 8:].any())
+        stats['snp_alt_aligned_channels_zero_in_golden'] += not any(g['nonzero'][8:])
       if not eq7 and len(mismatches) < 40:
-        bad = [c for c in range(7) if not np.array_equal(img[..., c], g[..., c])]
-        mismatches.append({'start': p.variant.start, 'alts': p.alt_combination, 'channels_differ': bad,
-                           'rows_ours': int(sum(1 for r in range(5, 100) if img[r].any())), 'rows_golden': int(sum(1 for r in range(5, 100) if g[r].any()))})
+        mismatches.append({'start': p.variant.start, 'alts': p.alt_combination, 'channels_differ': [c for c in range(7) if not same[c]],
+                           'rows_ours': o['rows'], 'rows_golden': g['rows']})
   stats['golden_examples'] = len(golden)
-  print(json.dumps(stats, indent=1))
-  print(json.dumps(mismatches[:10], indent=1))
-  with open(os.path.join(ROOT, 'tests/golden/pacbio_end_to_end_report.json'), 'w') as f:
-    json.dump({'stats': stats, 'first_mismatches': mismatches}, f, indent=1)
+  if write:
+    print(json.dumps(stats, indent=1))
+    print(json.dumps(mismatches[:10], indent=1))
+    with open(os.path.join(ROOT, 'tests/golden/pacbio_end_to_end_report.json'), 'w') as f:
+      json.dump({'stats': stats, 'first_mismatches': mismatches}, f, indent=1)
+  return stats
 
 
 if __name__ == '__main__':

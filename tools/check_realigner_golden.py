@@ -42,13 +42,15 @@ def decoded_features(e: dict) -> dict:
   return out
 
 
-def main(with_flags=False):
+def main(with_flags=False, td=T, bam_path=None, ref_path=None, shard_keys=None, write=True):
+  """Compares with the goldens in the testdata directory td; bam_path / ref_path default to its inputs, shard_keys (the
+  [start, alt allele indices] of each --task shard's examples) to its three shard files.  Returns the report."""
   from deepvariant_b200 import normalize_reads
   min_mapq = 1 if with_flags else 5
   examples_golden = 'golden.calling_examples.with_flags.tfrecord.gz' if with_flags else 'golden.calling_examples.tfrecord.gz'
-  golden_c = [] if with_flags else [cand.canonical_call(r) for r in tfrecord.read_records(T + 'golden.calling_candidates.tfrecord.gz')]
+  golden_c = [] if with_flags else [cand.canonical_call(r) for r in tfrecord.read_records(os.path.join(td, 'golden.calling_candidates.tfrecord.gz'))]
   golden_e, golden_features, golden_order = {}, {}, []
-  for r in tfrecord.read_records(T + examples_golden):
+  for r in tfrecord.read_records(os.path.join(td, examples_golden)):
     e = protos.parse_tf_example(r)
     v = protos.parse_variant(e['variant/encoded'][1][0])
     idx = tuple(protos.parse_alt_allele_indices(e['alt_allele_indices/encoded'][1][0]))
@@ -58,12 +60,15 @@ def main(with_flags=False):
   golden_shards = []
   for i in range(0 if with_flags else 3):
     keys = []
-    for r in tfrecord.read_records(T + f'golden.calling_examples.tfrecord.gz-0000{i}-of-00003'):
-      e = protos.parse_tf_example(r)
-      keys.append((protos.parse_variant(e['variant/encoded'][1][0]).start, tuple(protos.parse_alt_allele_indices(e['alt_allele_indices/encoded'][1][0]))))
+    if shard_keys is not None:
+      keys = [(k[0], tuple(k[1])) for k in shard_keys[i]]
+    else:
+      for r in tfrecord.read_records(os.path.join(td, f'golden.calling_examples.tfrecord.gz-0000{i}-of-00003')):
+        e = protos.parse_tf_example(r)
+        keys.append((protos.parse_variant(e['variant/encoded'][1][0]).start, tuple(protos.parse_alt_allele_indices(e['alt_allele_indices/encoded'][1][0]))))
     golden_shards.append(keys)
-  bam_path = T + 'input/NA12878_S1.chr20.10_10p1mb.bam'
-  ref = fasta.IndexedFastaReader(T + 'input/ucsc.hg19.chr20.unittest.fasta.gz')
+  bam_path = bam_path or os.path.join(td, 'input/NA12878_S1.chr20.10_10p1mb.bam')
+  ref = fasta.IndexedFastaReader(ref_path or os.path.join(td, 'input/ucsc.hg19.chr20.unittest.fasta.gz'))
   table = bam.NativeBamTable(bam_path, bam.ReadRequirements(min_mapping_quality=min_mapq))
   copts = cand.CandidateOptions(sample_name=cand.sample_name_from_bam(bam_path), small_model_vaf_context_window_size=51,
                                 min_mapping_quality=min_mapq, keep_legacy_allele_counter_behavior=with_flags)
@@ -135,11 +140,13 @@ def main(with_flags=False):
             'golden_only': sorted(k[0] for k in g_by if k not in o_by), 'ours_only': sorted(k[0] for k in o_by if k not in g_by),
             'golden_examples': len(golden_e), 'examples_planned': len(images), 'images_identical': len(img_eq),
             'golden_read_rows': rows_total, 'golden_read_rows_reproduced': rows_hit}
-  with open(os.path.join(ROOT, 'tests/golden/' + ('with_flags_golden_report.json' if with_flags else 'realigner_golden_report.json')), 'w') as f:
-    json.dump(report, f, indent=1)
-  print(json.dumps({k: v for k, v in report.items() if not isinstance(v, list) or len(v) < 20}, indent=1))
-  for p in partial[:10]:
-    print(p)
+  if write:
+    with open(os.path.join(ROOT, 'tests/golden/' + ('with_flags_golden_report.json' if with_flags else 'realigner_golden_report.json')), 'w') as f:
+      json.dump(report, f, indent=1)
+    print(json.dumps({k: v for k, v in report.items() if not isinstance(v, list) or len(v) < 20}, indent=1))
+    for p in partial[:10]:
+      print(p)
+  return report
 
 
 if __name__ == '__main__':
