@@ -2681,7 +2681,10 @@ int Plan(DvbCnn* net, const uint8_t* blob, int64_t blob_bytes) {
     const auto [Hin, Win] = hw[o.src];
     int Hout, Wout;
     if (o.same) { Hout = Hin; Wout = Win; }
-    else { Hout = (Hin - o.kh) / o.stride + 1; Wout = (Win - o.kw) / o.stride + 1; }
+    else {   // a window larger than the map has no output (C++ division truncates toward zero: (2 - 3) / 2 + 1 would be 1)
+      Hout = Hin < o.kh ? 0 : (Hin - o.kh) / o.stride + 1;
+      Wout = Win < o.kw ? 0 : (Win - o.kw) / o.stride + 1;
+    }
     if (Hout < 1 || Wout < 1) return dvb::fail(DVB_ERR_INVALID_ARGUMENT, "image %dx%d is too small for the network", net->H, net->W);
     hw[o.dst] = {Hout, Wout};
     if (merged_into[op_index] >= 0) continue;     // runs inside its group leader's GEMM
@@ -3302,18 +3305,37 @@ int Plan(DvbCnn* net, const uint8_t* blob, int64_t blob_bytes) {
     occ = std::max(1, std::min(occ, 512 / h.args.tmem_cols));
     h.ctas_per_nblock = std::max(1, net->num_sms * occ / h.args.n_blocks);
   }
-  if (EnvInt("DVB_CNN_LIST", 0))
-    for (size_t i = 0; i < net->convs.size(); ++i) {
-      const ConvLaunch& c = net->convs[i];
-      fprintf(stderr, "[conv %zu] %dx%d cin_blocks=%d bk=%d N=%d n_blocks=%d persist=%d pair=%d stages=%d\n", i, c.args.kh, c.args.kw, c.args.cin_blocks, c.args.block_k,
-              c.args.block_n, c.n_blocks, (int)c.persist, (int)c.pair, c.args.stages);
+  // Plan listing: which kernel runs each layer (dst = first tensor the step writes).  A [conv] line also gives the M tile box
+  // (Wt x Ht x Nt output pixels, flat = all pixels of the chunk in one row) and the M tile count at max_batch images.
+  if (EnvInt("DVB_CNN_LIST", 0)) {
+    fprintf(stderr, "[stem] %s\n", net->stem_rows ? "rows" : net->stem_fused ? "fused" : "patch");
+    for (size_t si = 0; si < net->steps.size(); ++si) {
+      const Step& stp = net->steps[si];
+      const char* dst = step_io[si].second[0].c_str();
+      if (stp.kind == 0) {
+        const ConvLaunch& c = net->convs[stp.index];
+        const ConvArgs& a = c.args;
+        const long m_tiles = c.flat ? ((long)net->max_batch * c.pixels_per_image + 127) / 128
+                                    : (long)a.tiles_w * a.tiles_h * ((net->max_batch + a.Nt - 1) / a.Nt);
+        fprintf(stderr, "[conv %d] %dx%d cin_blocks=%d bk=%d N=%d n_blocks=%d persist=%d pair=%d stages=%d dst=%s out=%dx%d box=%dx%dx%d flat=%d m_tiles=%ld\n",
+                stp.index, a.kh, a.kw, a.cin_blocks, a.block_k, a.block_n, c.n_blocks, (int)c.persist, (int)c.pair, a.stages, dst, a.Hout, a.Wout, a.Wt, a.Ht,
+                a.Nt, (int)c.flat, m_tiles);
+      } else if (stp.kind == 2) {
+        const HaloArgs& h = net->halos[stp.index].args;
+        fprintf(stderr, "[halo %d] %dx%d %dx%d cin_blocks=%d bk=%d N=%d n_blocks=%d P=%d Ht=%d T=%d nbuf=%d stages=%d n_split=%d smem=%d dst=%s\n", stp.index, h.kh,
+                h.kw, h.Hout, h.Wout, h.cin_blocks, h.block_k, h.block_n, h.n_blocks, h.P, h.Ht, h.T, h.nbuf, h.stages, h.n_split, net->halos[stp.index].smem, dst);
+      } else if (stp.kind == 3) {
+        const RowsArgs& r = net->rows[stp.index].args;
+        fprintf(stderr, "[rows %d] 3x3 %dx%d cout=%d pool=%d dst=%s\n", stp.index, r.Hout, r.Wout, r.cout, r.pool, dst);
+      } else {   // the kernel ForwardChunkLaunches picks for this pool (same switches, read again there)
+        const PoolLaunch& p = net->pools[stp.index];
+        const char* kernel = p.mode == 0 ? (!p.in_res && EnvInt("DVB_CNN_MAXPOOL_H2", 1) ? "maxpool3x3s2_h2" : "pool3x3")
+                                         : (!p.in_res && p.Hout == p.Hin && p.Wout == p.Win && EnvInt("DVB_CNN_AVGPOOL_FLAT", 1) ? "avgpool3x3s1" : "pool3x3");
+        fprintf(stderr, "[pool %d] %s %dx%d -> %dx%d bias=%d kernel=%s dst=%s\n", stp.index, p.mode ? "avg" : "max", p.Hin, p.Win, p.Hout, p.Wout,
+                (int)(p.bias != nullptr), kernel, dst);
+      }
     }
-  if (EnvInt("DVB_CNN_LIST", 0))
-    for (size_t i = 0; i < net->halos.size(); ++i) {
-      const HaloArgs& h = net->halos[i].args;
-      fprintf(stderr, "[halo %zu] %dx%d %dx%d cin_blocks=%d bk=%d N=%d n_blocks=%d P=%d Ht=%d T=%d nbuf=%d stages=%d n_split=%d smem=%d\n", i, h.kh, h.kw, h.Hout, h.Wout,
-              h.cin_blocks, h.block_k, h.block_n, h.n_blocks, h.P, h.Ht, h.T, h.nbuf, h.stages, h.n_split, net->halos[i].smem);
-    }
+  }
   if (cudaDeviceSynchronize() != cudaSuccess) return dvb::fail(DVB_ERR_CUDA, "weight upload failed: %s", cudaGetErrorString(cudaGetLastError()));
   return DVB_OK;
 }
